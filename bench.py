@@ -6,6 +6,7 @@
     python bench.py --workload infer --batch {1,16} [--frames 400]      # configs[3]: Flowtron.infer, frames/s + RTF
     python bench.py --workload mel [--utterances 10000]                 # configs[4]: TacotronSTFT sweep, GB/s vs HBM
     python bench.py --impl reference [--workload ...]                   # the UNMODIFIED reference on the host CPU cores
+    python bench.py ... --dump-outputs DIR                              # also write the last timed step's outputs as DIR/<name>.npy
 
 train: a step = Flowtron.forward -> FlowtronLoss -> backward -> bucketed NCCL gradient all-reduce (N>1) -> grad-norm clip
 -> RAdam step (train.py:281-331).  `value` = valid mel frames (sum of out_lens over all ranks) per second with inputs
@@ -52,7 +53,38 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--streams", type=int, default=1, help="train: 2 = two half-batch pipelines on two CUDA streams")
     ap.add_argument("--profile", action="store_true", help="short run for ncu: no e2e leg, no CPU baseline, no graph, warm-up as given")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path computed in its last timed step as DIR/<name>.npy (float32, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the b200 implementation's outputs")
+    return args
+
+
+# ------------------------------------------------------------------------------------------------ output dump
+DUMP_MAX_ELEMS = 1 << 20        # per array; larger outputs are represented by a fixed, seeded sample of their elements
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(outdir, arrays):
+    """Write {name: tensor} as outdir/<name>.npy in float32.  An array of more than DUMP_MAX_ELEMS elements is flattened and
+    sampled at DUMP_MAX_ELEMS positions drawn from a generator seeded with 0, so two builds run with the same arguments
+    write the same positions and can be compared element for element."""
+    import numpy as np
+    os.makedirs(outdir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_MAX_ELEMS:
+            g = torch.Generator().manual_seed(0)
+            idx = torch.randint(0, t.numel(), (DUMP_MAX_ELEMS,), generator=g).sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        a = t.float().cpu().numpy()
+        total += a.nbytes
+        assert total <= DUMP_MAX_BYTES, f"output dump exceeds {DUMP_MAX_BYTES} bytes"
+        np.save(os.path.join(outdir, f"{name}.npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------ clocks
@@ -259,6 +291,7 @@ def run_train(args):
             opt.zero_grad(set_to_none=True)
 
     loss_static = torch.zeros((), device=dev)
+    last = {}                                                 # the latest step's outputs (under the graph: its static outputs)
 
     def step_body(d):
         zero_grads()
@@ -272,6 +305,8 @@ def run_train(args):
             torch.nn.utils.clip_grad_norm_(model.parameters(), 1.0, foreach=True)
         opt.step()
         loss_static.copy_(loss.detach())
+        last.update(out=[[t.detach() for t in x] if isinstance(x, list) else x.detach() for x in out[:4]], nll=nll.detach(),
+                    gate_loss=gl.detach())
 
     n_warm = args.warmup if args.profile else max(3, args.warmup)
     _lib.reset_launch_count()
@@ -345,6 +380,8 @@ def run_train(args):
     sampler = ClockSampler(local)
     sampler.start()
     ms = timed(step_value, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, train_outputs(model, last, static, loss_static))
     ms_e2e = ms
     if not args.profile:
         for s in range(2):
@@ -423,6 +460,24 @@ def run_train(args):
     print(json.dumps(out))
 
 
+def train_outputs(model, last, d, loss):
+    """What a caller of one training step receives: the losses, the forward outputs at valid positions (pads are not
+    defined), and the parameters and gradients the step left behind."""
+    z, log_s_list, gate, attns = last["out"]
+    T = z.size(0)
+    valid = torch.arange(T, device=z.device)[:, None] < d["out_lens"][None, :]                       # [T, B]
+    text_valid = torch.arange(attns[0].size(2), device=z.device)[None, :] < d["in_lens"][:, None]     # [B, L]
+    attn_valid = valid.t()[:, :, None] & text_valid[:, None, :]                                        # [B, T, L]
+    res = {"loss": loss, "nll": last["nll"], "gate_loss": last["gate_loss"], "z": z[valid], "gate": gate[valid]}
+    for i, (ls, at) in enumerate(zip(log_s_list, attns)):
+        res[f"log_s_{i}"] = ls[valid]
+        res[f"attn_{i}"] = at[attn_valid]
+    params = list(model.parameters())
+    res["params"] = torch.cat([p.detach().reshape(-1) for p in params])
+    res["grads"] = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).detach().reshape(-1) for p in params])
+    return res
+
+
 # ------------------------------------------------------------------------------------------------ infer
 def run_infer(args):
     from flowtron_b200 import _lib, synth
@@ -448,10 +503,12 @@ def run_infer(args):
     spk_h = torch.zeros(B, dtype=torch.long).pin_memory()
     res, text, spk = res_h.to(dev), text_h.to(dev), spk_h.to(dev)
     out_h = torch.empty(B, 80, T).pin_memory()
+    last = {}
 
     def step():
         with torch.no_grad():
-            mel, _ = model.infer(res, spk, text, temperature=1.0, gate_threshold=0.5)
+            mel, attns = model.infer(res, spk, text, temperature=1.0, gate_threshold=0.5)
+        last.update(mel=mel, attns=attns)
         return mel
 
     def step_e2e():
@@ -473,6 +530,8 @@ def run_infer(args):
     launches = _lib.launch_count()
     trep = _lib.timing_report()
     _lib.timing(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"mel": last["mel"], **{f"attn_{i}": torch.stack(a) for i, a in enumerate(last["attns"])}})
     ms_e2e = ms if args.profile else timed(step_e2e, args.steps)
     clocks = sampler.stop()
     if rank != 0:
@@ -552,6 +611,8 @@ def run_mel(args):
     launches = _lib.launch_count()
     trep = _lib.timing_report()
     _lib.timing(False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"mel": out})
     ms_e2e = ms
     h2d = d2h = 0
     if not args.profile:
@@ -605,6 +666,9 @@ def run_mel(args):
 
 def main():
     args = parse()
+    # the training step's dropout masks derive from torch's global seed, which is otherwise drawn at random per process:
+    # fix it so that runs with the same arguments compute on identical inputs
+    torch.manual_seed(1234)
     if args.impl == "reference":
         return run_reference_arm(args)
     if args.workload == "train":

@@ -1,6 +1,6 @@
 """CPU restatement of the reference's data-layer pieces that sit next to the hot path (TEST INFRASTRUCTURE):
 beta_binomial_prior_distribution (data.py:31-41) and DataCollate.__call__ (data.py:197-246).  Pinned against the
-reference's own functions in tests/test_oracle_data.py (build container, `needs_reference`)."""
+reference's own outputs (tests/golden/data_collate.npz, written by tests/make_golden.py) in tests/test_oracle_data.py."""
 from __future__ import annotations
 
 import numpy as np

@@ -1,7 +1,7 @@
-"""Import the UNMODIFIED reference modules on CPU: from /root/reference in the build container (used by
-tests/make_golden.py to generate fixtures and by tests marked ``needs_reference``), or from their byte-compiled staging
-in oracle/_ref/ (oracle/build_ref.py) on the GPU box, where ONLY bench.py's reference arm / cpu_baseline leg may use it
-(nothing in ``-m gpu`` tests or smoke() reads the reference).  Shims (SURVEY.md §8c / Appendix B):
+"""Import the UNMODIFIED reference modules on CPU: from the reference tree (``FLOWTRON_REFERENCE``; used by
+tests/make_golden.py to generate the fixtures the tests compare against), or from their byte-compiled staging in
+oracle/_ref/ (oracle/build_ref.py), which ONLY bench.py's reference arm / cpu_baseline leg may use (no test and not
+smoke() reads the reference).  Shims (SURVEY.md §8c / Appendix B):
   1. flowtron.get_mask_from_lengths hard-codes torch.cuda.LongTensor (flowtron.py:48) -> arange version;
   2. AR_Step.infer allocates torch.cuda.FloatTensor (flowtron.py:785) -> alias to torch.FloatTensor;
   3. audio_processing imports librosa (absent here) -> stub providing filters.mel / util.pad_center /

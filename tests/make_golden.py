@@ -139,6 +139,67 @@ def radam_case():
     print("radam: 9 steps recorded")
 
 
+def host_layer_cases():
+    """Reference outputs the CPU restatements of the data layer, the STFT and the forced-alignment infer branch are pinned
+    against (tests/test_oracle_data.py, tests/test_abi_and_host.py), with the inputs that produced them."""
+    import types
+    cwd = os.getcwd()
+    os.chdir(ref_shims.REF)                                 # text/__init__ opens data/cmudict_dictionary relative to the cwd
+    try:
+        ref_shims.import_audio_processing()                 # librosa stub before data.py imports audio_processing
+        for name in ("unidecode", "inflect"):                # text-cleaning dependencies (absent here, unused by the collate)
+            if name not in sys.modules:
+                m = types.ModuleType(name)
+                m.unidecode = lambda s: s
+                m.engine = lambda: None
+                sys.modules[name] = m
+        sys.path.insert(0, ref_shims.REF)
+        import data as RD
+    finally:
+        os.chdir(cwd)
+    rec = {"prior_11_29": RD.beta_binomial_prior_distribution(11, 29, 1.0).numpy()}
+    g = torch.Generator().manual_seed(0)
+    batch = []
+    for i, (F_, P_) in enumerate([(29, 11), (40, 17), (5, 17), (33, 3)]):
+        item = (torch.randn(80, F_, generator=g), torch.LongTensor([F_ % 3]), torch.randint(1, 100, (P_,), generator=g),
+                RD.beta_binomial_prior_distribution(P_, F_, 1.0))
+        batch.append(item)
+        for k, t in zip(("mel", "speaker", "text", "prior"), item):
+            rec[f"in_{k}_{i}"] = t.numpy()
+    for i, t in enumerate(RD.DataCollate(1, use_attn_prior=True)(batch)):
+        rec[f"collate_{i}"] = t.numpy()
+    np.savez_compressed(os.path.join(OUT, "data_collate.npz"), **rec)
+
+    AP = ref_shims.import_audio_processing()
+    g = torch.Generator().manual_seed(3)
+    y = torch.rand(2, 3000, generator=g) * 1.9 - 0.95
+    m, p = AP.STFT(1024, 256, 1024).transform(y)
+    np.savez_compressed(os.path.join(OUT, "stft_transform.npz"), y=y.numpy(), magnitude=m.numpy(), phase=p.numpy())
+
+    # AR_Step.infer / AR_Back_Step.infer with `attns` given (flowtron.py:585-588, 797)
+    cfg = dict(synth.DEFAULT_MODEL_CONFIG, n_flows=2, use_gate_layer=False)
+    F, model = ref_shims.reference_model(cfg, synth.synth_params(cfg, 17))
+    g = torch.Generator().manual_seed(2)
+    T, L = 10, 6
+    residual = torch.randn(T, 1, 80, generator=g) * 0.5
+    enc = torch.randn(L, 1, 640, generator=g)
+    attns = torch.softmax(torch.randn(T, L, generator=g), -1)
+    with torch.no_grad():
+        r0, _ = model.flows[0].infer(residual, enc, attns)
+        r1, _ = model.flows[1].infer(residual, enc, attns)
+    np.savez_compressed(os.path.join(OUT, "ar_step_forced_attns.npz"), seed=np.int64(17), residual=residual.numpy(),
+                        enc=enc.numpy(), attns=attns.numpy(), flow0=r0.numpy(), flow1=r1.numpy())
+
+    # the reference's state_dict layout for the default config: key order and shapes
+    cfg = dict(synth.DEFAULT_MODEL_CONFIG)
+    F, model = ref_shims.reference_model(cfg, synth.synth_params(cfg, 5))
+    sd = model.state_dict()
+    rec = {"keys": np.array(list(sd.keys()))}
+    rec.update({f"shape::{k}": np.array(v.shape, dtype=np.int64) for k, v in sd.items()})
+    np.savez_compressed(os.path.join(OUT, "state_dict_layout.npz"), **rec)
+    print("host layer: data_collate, stft_transform, ar_step_forced_attns, state_dict_layout")
+
+
 def big_cases():
     """BASELINE-shape fixtures (VERDICT r1 #1): a T=1000 training step (cfg 2 shapes at the largest B the CPU reference
     finishes in minutes) and cfg-4 inference requests (T=400 default, T=1000), all 2-flow."""
@@ -163,12 +224,15 @@ def main():
     infer_case("b4nogate", n_flows=2, B=4, T=32, L=16, seed=8, gate_bias=0.0, use_gate=False)
     mel_case()
     radam_case()
+    host_layer_cases()
     big_cases()
 
 
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "radam":     # regenerate only the optimizer fixture
         radam_case()
+    elif len(sys.argv) > 1 and sys.argv[1] == "host":    # only the data-layer / STFT / forced-alignment / layout fixtures
+        host_layer_cases()
     elif len(sys.argv) > 1 and sys.argv[1] == "ctc":     # only the CTC-loss fixture
         torch.manual_seed(0)
         torch.set_num_threads(8)

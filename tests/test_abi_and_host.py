@@ -4,10 +4,11 @@ import ctypes
 import os
 import re
 
+import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import GOLDEN, ROOT
 from flowtron_b200 import synth
 
 
@@ -37,18 +38,21 @@ def test_state_dict_layout_matches_reference_spec():
         m.load_state_dict(synth.synth_params(cfg, 3), strict=True)
 
 
-@pytest.mark.needs_reference
 def test_state_dict_loads_into_reference_and_back():
-    from oracle import ref_shims
-    if not ref_shims.available():
-        pytest.skip("no /root/reference here")
+    """Against the reference model's state_dict layout for the default config (key order and shapes, written by
+    tests/make_golden.py): a reference checkpoint loads strictly into ours, and ours has exactly its keys and shapes."""
     from flowtron_b200.flowtron import Flowtron
+    gold = np.load(os.path.join(GOLDEN, "state_dict_layout.npz"), allow_pickle=False)
+    ref_keys = [str(k) for k in gold["keys"]]
+    ref_sd = {k: torch.zeros(tuple(int(d) for d in gold[f"shape::{k}"])) for k in ref_keys}
     cfg = dict(synth.DEFAULT_MODEL_CONFIG)
-    F, ref = ref_shims.reference_model(cfg, synth.synth_params(cfg, 5))
     ours = Flowtron(**cfg)
-    ours.load_state_dict(ref.state_dict(), strict=True)
-    ref.load_state_dict(ours.state_dict(), strict=True)
-    assert list(ours.state_dict().keys()) == list(ref.state_dict().keys())
+    ours.load_state_dict(synth.synth_params(cfg, 5), strict=True)
+    ours.load_state_dict(ref_sd, strict=True)
+    sd = ours.state_dict()
+    assert list(sd.keys()) == ref_keys
+    for k, v in sd.items():
+        assert tuple(v.shape) == tuple(ref_sd[k].shape), k
 
 
 def test_product_path_fails_loudly_on_cpu():

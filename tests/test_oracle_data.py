@@ -1,14 +1,19 @@
 """CPU: pin the data-layer restatements (oracle/data_oracle.py, oracle/stft_oracle.stft_transform, and the closed-form
-prior the product's synthetic batches use) against the reference's own functions (build container only) and against
-scipy's beta-binomial everywhere."""
+prior the product's synthetic batches use) against outputs of the reference's own functions (fixtures written by
+tests/make_golden.py) and against scipy's beta-binomial."""
+import os
+
 import numpy as np
-import pytest
 import torch
 
+from conftest import GOLDEN
 from oracle import data_oracle as D
-from oracle import ref_shims
 from flowtron_b200 import synth
 from oracle import stft_oracle as S
+
+
+def _load(name):
+    return dict(np.load(os.path.join(GOLDEN, name), allow_pickle=False))
 
 
 def test_closed_form_prior_equals_scipy_loop():
@@ -19,63 +24,35 @@ def test_closed_form_prior_equals_scipy_loop():
         assert np.abs(a - b).max() <= 1e-12 + 1e-9 * np.abs(b).max()
 
 
-@pytest.mark.needs_reference
-@pytest.mark.skipif(not ref_shims.available(), reason="needs /root/reference")
-def test_data_oracle_matches_reference_data_py(monkeypatch):
-    monkeypatch.chdir(ref_shims.REF)                         # text/__init__ opens data/cmudict_dictionary relative to the cwd
-    ref_shims.import_audio_processing()                     # librosa stub before data.py imports audio_processing
-    import sys
-    import types
-    for name in ("unidecode", "inflect"):                    # text-cleaning dependencies (absent here, unused by the collate)
-        if name not in sys.modules:
-            m = types.ModuleType(name)
-            m.unidecode = lambda s: s
-            m.engine = lambda: None
-            sys.modules[name] = m
-    sys.path.insert(0, ref_shims.REF)
-    import data as RD
-    p_ref = RD.beta_binomial_prior_distribution(11, 29, 1.0)
+def test_data_oracle_matches_reference_data_py():
+    gold = _load("data_collate.npz")
+    p_ref = torch.from_numpy(gold["prior_11_29"])
     assert torch.equal(p_ref, D.beta_binomial_prior_distribution(11, 29, 1.0))
-    g = torch.Generator().manual_seed(0)
-    batch = []
-    for F_, P_ in [(29, 11), (40, 17), (5, 17), (33, 3)]:
-        batch.append((torch.randn(80, F_, generator=g), torch.LongTensor([F_ % 3]), torch.randint(1, 100, (P_,), generator=g),
-                      RD.beta_binomial_prior_distribution(P_, F_, 1.0)))
-    ref = RD.DataCollate(1, use_attn_prior=True)(batch)
+    batch = [tuple(torch.from_numpy(gold[f"in_{k}_{i}"]) for k in ("mel", "speaker", "text", "prior")) for i in range(4)]
+    ref = [torch.from_numpy(gold[f"collate_{i}"]) for i in range(7)]
     mine = D.collate(batch, 1, use_attn_prior=True)
+    assert len(mine) == len(ref)
     for a, b in zip(ref, mine):
         assert a.shape == b.shape and torch.equal(a.float(), b.float())
 
 
-@pytest.mark.needs_reference
-@pytest.mark.skipif(not ref_shims.available(), reason="needs /root/reference")
 def test_stft_transform_oracle_matches_reference():
-    AP = ref_shims.import_audio_processing()
-    stft = AP.STFT(1024, 256, 1024)
-    g = torch.Generator().manual_seed(3)
-    y = torch.rand(2, 3000, generator=g) * 1.9 - 0.95
-    m_ref, p_ref = stft.transform(y)
-    m, p = S.stft_transform(y)
+    gold = _load("stft_transform.npz")
+    m_ref, p_ref = torch.from_numpy(gold["magnitude"]), torch.from_numpy(gold["phase"])
+    m, p = S.stft_transform(torch.from_numpy(gold["y"]))
     assert torch.allclose(m, m_ref, atol=1e-6) and torch.allclose(p, p_ref, atol=1e-6)
 
 
-@pytest.mark.needs_reference
-@pytest.mark.skipif(not ref_shims.available(), reason="needs /root/reference")
 def test_forced_alignment_branch_matches_reference_ar_step_infer():
     """AR_Step.infer / AR_Back_Step.infer with `attns` given (flowtron.py:585-588, 797): oracle vs the reference modules.
     (Flowtron.infer itself cannot be driven with attns in the reference: `reversed(attns)[i]` at :924 raises.)"""
     from oracle import flowtron_oracle as O
+    gold = _load("ar_step_forced_attns.npz")
     cfg = dict(synth.DEFAULT_MODEL_CONFIG, n_flows=2, use_gate_layer=False)
-    params = synth.synth_params(cfg, 17)
-    F, model = ref_shims.reference_model(cfg, params)
-    g = torch.Generator().manual_seed(2)
-    T, L = 10, 6
-    residual = torch.randn(T, 1, 80, generator=g) * 0.5
-    enc = torch.randn(L, 1, 640, generator=g)
-    attns = torch.softmax(torch.randn(T, L, generator=g), -1)
+    params = synth.synth_params(cfg, int(gold["seed"]))
+    residual, enc, attns = (torch.from_numpy(gold[k]) for k in ("residual", "enc", "attns"))
+    r0, r1 = torch.from_numpy(gold["flow0"]), torch.from_numpy(gold["flow1"])
     with torch.no_grad():
-        r0, _ = model.flows[0].infer(residual, enc, attns)
-        r1, _ = model.flows[1].infer(residual, enc, attns)
         o0, _ = O.ar_step_infer(params, O.flow_prefix(0), residual, enc, attns=attns)
         o1, _ = O.ar_back_step_infer(params, "flows.1", residual, enc, attns=attns)
     assert (r0 - o0).abs().max().item() <= 1e-5 * r0.abs().max().item()
