@@ -4,7 +4,8 @@ Functional style: every function takes ``p``, a flat ``{state_dict key: tensor}`
 dict in the reference's checkpoint layout (SURVEY.md §8a row 15), so the same
 weights drive the reference, this oracle and the CUDA path.  Everything is
 ordinary differentiable torch, so ``torch.autograd`` of these functions is the
-gradient oracle as well.
+gradient oracle as well.  They compute in the dtype of their inputs: given float64
+tensors they are a float64 reference (tests/test_gpu_flow_step.py).
 
 Each function cites the reference lines it restates (paths relative to
 /root/reference).  Pinned against reference-generated fixtures by
@@ -108,13 +109,13 @@ def attention_forward(p: Params, pre: str, queries: Tensor, text: Tensor, mask: 
             e = e.masked_fill(mask.transpose(1, 2), -float("inf"))   # :574-576
         a = torch.softmax(e, dim=2)                              # :577
         if attn_prior is not None:
-            lp = torch.log(a.float() + 1e-20) + torch.log(attn_prior.float() + 1e-20)  # :546-548
+            lp = torch.log(a + 1e-20) + torch.log(attn_prior.to(a.dtype) + 1e-20)  # :546-548
             attn_logprob = lp.clone()                            # :550 (before masking)
             if mask is not None:
                 lp = lp.masked_fill(mask.transpose(1, 2), -float("inf"))
             a = torch.softmax(lp, dim=2)                         # :556
         else:
-            attn_logprob = torch.log(a.float() + 1e-8)           # :583
+            attn_logprob = torch.log(a + 1e-8)                   # :583
     else:
         a = attn
         attn_logprob = None
@@ -356,7 +357,7 @@ def flowtron_loss(model_output, gate_target: Tensor, in_lens: Tensor, out_lens: 
                   sigma: float = 1.0, gate_loss: bool = True):
     """FlowtronLoss.forward default branch (no GMM, no CTC), flowtron.py:200-243 (Appendix A.5)."""
     z, log_s_list, gate_pred = model_output[0], model_output[1], model_output[2]
-    mask = get_mask_from_lengths(out_lens, z.shape[0]).transpose(0, 1)[..., None].float()
+    mask = get_mask_from_lengths(out_lens, z.shape[0]).transpose(0, 1)[..., None].to(z.dtype)
     n = mask.sum()
     log_s_total = sum(torch.sum(ls * mask) for ls in log_s_list)
     zm = z * mask
@@ -364,7 +365,7 @@ def flowtron_loss(model_output, gate_target: Tensor, in_lens: Tensor, out_lens: 
     gl = torch.zeros(1)
     if gate_loss and gate_pred is not None:
         gp = (gate_pred * mask)[..., 0].permute(1, 0)
-        gl = F.binary_cross_entropy_with_logits(gp, gate_target, reduction="none")
+        gl = F.binary_cross_entropy_with_logits(gp, gate_target.to(gp.dtype), reduction="none")
         gl = (gl.permute(1, 0) * mask[:, :, 0]).sum() / n
     return nll, gl
 

@@ -243,6 +243,7 @@ def test_batch_above_32_uses_the_wide_paths_and_matches_split_runs():
 
     def run(sl):
         model = build_model(cfg, 43)
+        model.max_kernel_batch = 64          # the default (32) would run B = 40 as a 32- and an 8-utterance launch
         model.train()
         model.encoder.p_dropout = 0.0
         Lp = int(cu["in_lens"][sl].max())

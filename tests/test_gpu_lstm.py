@@ -36,8 +36,26 @@ def _oracle(xproj, whh, lens):
     return out, torch.stack(cs)
 
 
-@pytest.mark.parametrize("T,B,lens", [(6, 2, None), (40, 5, [40, 3, 17, 40, 1]), (33, 32, "rand"), (20, 48, "rand")])
+# B = 1 (one 8-row batch box), B = 33 (the smallest batch past the cluster BPTT: Bbox 40), B = 64 (the widest launch), T = 1
+@pytest.mark.parametrize("T,B,lens", [(6, 2, None), (40, 5, [40, 3, 17, 40, 1]), (33, 32, "rand"), (20, 48, "rand"),
+                                      (1, 1, None), (17, 1, None), (1, 33, None), (9, 33, "rand"), (1, 64, None),
+                                      (12, 64, "rand")])
 def test_lstm_fwd_bwd(T, B, lens):
+    _check_lstm(T, B, lens)
+
+
+# The 64-CTA forward (16 units per CTA instead of 8) that Flowtron.forward selects for two concurrent half batches
+@pytest.mark.parametrize("T,B,lens", [(1, 1, None), (40, 5, [40, 3, 17, 40, 1]), (33, 32, "rand")])
+def test_lstm_fwd_bwd_64cta_forward(T, B, lens):
+    from flowtron_b200 import _lib
+    _lib.set_lstm_half_sm(True)
+    try:
+        _check_lstm(T, B, lens)
+    finally:
+        _lib.set_lstm_half_sm(False)
+
+
+def _check_lstm(T, B, lens):
     from flowtron_b200 import _lib
     xproj, whh = _mk(T, B, T * 100 + B, wscale=2.0)
     if lens == "rand":
@@ -55,12 +73,16 @@ def test_lstm_fwd_bwd(T, B, lens):
     hseq = torch.zeros(T, B, H + 64, device=dev, dtype=torch.float16)[:, :, :H]   # strided view like d[T,B,1664]
     gates = torch.zeros(T, B, 4 * H, device=dev, dtype=torch.float16)
     cst = torch.zeros(T, B, H, device=dev)
+    h32 = torch.full((T, B, H + 32), float("nan"), device=dev)[:, :, :H]      # fp32 copy of h, strided like hseq
     lens_d = None if lens_t is None else lens_t.to(dev, torch.int32)
-    _lib.lstm_fwd(xproj.to(dev), whh.to(dev).half(), lens_d, hseq, gates, cst)
+    _lib.lstm_fwd(xproj.to(dev), whh.to(dev).half(), lens_d, hseq, gates, cst, h32)
     torch.cuda.synchronize()
     assert _lib.device_status() == 0
     err = (hseq.float().cpu() - ref_h.detach()).abs().max().item()
     assert err < 3e-3, err
+    err32 = (h32.cpu() - ref_h.detach()).abs().max().item()
+    assert err32 < 3e-3, err32
+    assert (h32.half() == hseq).all()                                          # hseq is h32 rounded to fp16
     vm = torch.ones(T, B, dtype=torch.bool) if lens_t is None else (torch.arange(T)[:, None] < lens_t[None, :])
     cerr = (cst.cpu() - ref_c.detach())[vm].abs().max().item()
     assert cerr < 5e-3, cerr
